@@ -239,6 +239,46 @@ def sharded_parity(mode, k, n, counts, sums, tsc, g_counts, g_sums, merged_score
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, res, mode: int):
+    """what a caller of the timed path receives from its last step, as float64 .npy files (exact for docIDs, counts and 32-bit halves of
+    the checksums): per-query match counts and docID checksums, and the matched docIDs themselves, or a fixed seeded sample of their
+    positions in the concatenated result when they exceed DUMP_BYTES; top-k mode: the [nq, k] docIDs and scores (-1 = no entry)"""
+    import trinity_b200 as tb
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    counts = np.asarray(res.match_counts[: res.nq], np.uint64)
+    np.save(d / "match_counts.npy", counts.astype(np.float64))
+    if mode == tb.MODE_SCORED_TOPK:
+        ids, sc = np.full((res.nq, res.k), -1.0), np.full((res.nq, res.k), -1.0)
+        for q in range(res.nq):
+            qd, qs = res.query(q)
+            ids[q, : len(qd)], sc[q, : len(qs)] = qd, qs
+        np.save(d / "topk_docids.npy", ids)
+        np.save(d / "topk_scores.npy", sc)
+        return
+    sums = res.checksums()
+    np.save(d / "docid_checksums_hi.npy", (sums >> np.uint64(32)).astype(np.float64))
+    np.save(d / "docid_checksums_lo.npy", (sums & np.uint64(0xFFFFFFFF)).astype(np.float64))
+    total = int(counts.sum())
+    cap = (DUMP_BYTES - 64 * res.nq) // 16   # sampled docIDs and their positions, 8 bytes each
+    pos = np.arange(total, dtype=np.int64) if total <= cap else np.sort(np.random.default_rng(0x5EED).choice(total, cap, replace=False))
+    out = np.empty(len(pos), np.float64)
+    ends = np.cumsum(counts.astype(np.int64))
+    buf = np.empty(max(1, int(counts.max()) if res.nq else 1), np.uint32)
+    lo = 0
+    for q in range(res.nq):
+        hi = int(np.searchsorted(pos, ends[q]))
+        if hi > lo:
+            qd = res.query(q)[0] if res.docids is not None else res.decode_query(q, buf)
+            out[lo:hi] = qd[pos[lo:hi] - (ends[q] - int(counts[q]))]
+        lo = hi
+    np.save(d / "docids.npy", out)
+    np.save(d / "docids_position.npy", pos.astype(np.float64))
+
+
 def reference_sample(r, texts, scored, k, cores, budget_s):
     """run the reference's exec_query over a prefix of the batch sized by a probe for ~budget_s of host time"""
     probe = min(len(texts), 64)
@@ -308,7 +348,7 @@ class Job:
                                                     a.ndocs, synth.sum_hits), synth)
         return self.refs[codec][0]
 
-    def run(self, workload: str, K: int, W: int, cpu_budget_s: float, with_clocks: bool) -> dict:
+    def run(self, workload: str, K: int, W: int, cpu_budget_s: float, with_clocks: bool, dump_dir: str | None = None) -> dict:
         import trinity_b200 as tb
         from trinity_b200.sharded import device_view
         torch, dist, args, world, rank = self.torch, self.dist, self.args, self.world, self.rank
@@ -388,6 +428,8 @@ class Job:
         torch.cuda.synchronize()
         e2e_s = time.perf_counter() - t0
         clocks = sampler.stop() if sampler else None
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, res, emode)
         # the same end-to-end step with plain 32-bit docIDs out (TRN_MODE_DOCS_ONLY), for comparison with the compact encoding
         plain = None
         if emode != mode:
@@ -467,7 +509,9 @@ class Job:
             line["clocks"] = clocks
 
         # ---------------- reference leg: CPU baseline + full-size parity (rank 0 runs the reference; every rank contributes its results)
-        if not args.no_cpu_baseline:
+        if not args.no_cpu_baseline and not (ROOT / "oracle" / "_ref" / "libtrinity_ref.so").exists():
+            line["cpu_baseline"] = line["parity"] = {"skipped": "oracle/_ref (the reference's own code) is not built"}
+        elif not args.no_cpu_baseline:
             g_counts = g_sums = m_scores = None
             if world > 1:
                 # per-query match counts + docID checksums of THIS rank's shard, summed over ranks (uint64 arithmetic, wrap-around is fine)
@@ -527,6 +571,7 @@ def main():
                          "replayed by trn_result_decode) or plain 32-bit docIDs (TRN_MODE_DOCS_ONLY)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the primary workload's results of the last timed step to DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -537,7 +582,7 @@ def main():
         return reference_arm(args, rank, world, K, W)
 
     job = Job(args)
-    line = job.run(args.workload, K, W, cpu_budget_s=30.0, with_clocks=True)
+    line = job.run(args.workload, K, W, cpu_budget_s=30.0, with_clocks=True, dump_dir=args.dump_outputs)
     line["numa"] = job.numa
     subs = []
     if args.sub == "auto":

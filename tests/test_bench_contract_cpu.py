@@ -11,7 +11,7 @@ ROOT = Path(__file__).resolve().parent.parent
 
 
 @pytest.mark.parametrize("workload", ["and2", "or10"])
-def test_reference_arm_prints_the_contract_line(ref, workload):
+def test_reference_arm_prints_the_contract_line(real_ref, workload):
     p = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--workload", workload, "--ndocs", "200000", "--nterms", "64",
                         "--nq", "16", "--steps", "1", "--warmup", "1"], capture_output=True, text=True, timeout=600)
     assert p.returncode == 0, p.stderr[-2000:]
@@ -69,7 +69,7 @@ def test_full_size_parity_checker_is_exact_in_uint64(ref):
     assert bench.full_size_parity(res, tb.MODE_DOCS_ONLY, 100, res.match_counts, sums, None, None, 2)["docid_checksums_equal"] is False
 
 
-def test_reference_side_binding_fails_loudly_without_a_gpu(ref):
+def test_reference_side_binding_fails_loudly_without_a_gpu(real_ref):
     """oracle/_ref/libtrinity_ref_gpu.so = the reference + integration/gpu_exec.cpp: attaching the device twin of an index source needs
     a CUDA device; without one it reports the engine's error (no silent CPU detour), and the library's exec_query() keeps using the
     reference's own span for sources that have no twin"""

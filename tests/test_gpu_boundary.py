@@ -16,6 +16,14 @@ from test_gpu_parity import TEMPLATES
 from util import assert_close_scores, assert_same_docs, closed_form_lists
 
 pytestmark = pytest.mark.gpu
+
+
+@pytest.fixture
+def ref(real_ref):
+    """these tests run the reference's own code, not its recorded outputs"""
+    return real_ref
+
+
 NDOCS = 400_000
 
 

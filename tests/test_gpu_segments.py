@@ -8,6 +8,14 @@ from trinity_b200.segments import SegmentCollection
 from util import assert_close_scores, assert_same_docs, assert_topk_equal
 
 pytestmark = pytest.mark.gpu
+
+
+@pytest.fixture
+def ref(real_ref):
+    """these tests run the reference's own code, not its recorded outputs"""
+    return real_ref
+
+
 NDOCS = 200_000
 QUERIES = ["w1 AND w2", "w3 OR w7 OR w9", "w1 AND (w2 OR w3) NOT w5", "w10", "(w1 AND w2) OR (w3 AND w4)", "w2 AND onlyold", "w1 OR onlynew",
            "missing AND w1", "missing OR w4"]

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 import trinity_b200 as tb
-from refharness import load_ref
+from refharness import load_golden_ref
 
 
 ERASED = np.array([3, 17, 4000, 40000, 70001, 1 << 20], np.uint32)  # a session cannot erase a document it also indexes
@@ -27,8 +27,8 @@ def make_lists(seed, nterms=40, ndocs=6000):
 
 @pytest.mark.parametrize("codec", [0, 1])
 def test_segment_reader_matches_reference(tmp_path, codec):
-    ref = load_ref()
-    lists = make_lists(7 + codec)
+    ref = load_golden_ref()
+    lists = make_lists(7 + codec, ndocs=1500)   # the segment directories it reads are stored in tests/golden: keep them small
     erased = ERASED
     path = tmp_path / "100"
     path.mkdir()
@@ -51,7 +51,7 @@ def test_segment_reader_matches_reference(tmp_path, codec):
 
 
 def test_segment_without_updates_and_errors(tmp_path):
-    ref = load_ref()
+    ref = load_golden_ref()
     path = tmp_path / "7"
     path.mkdir()
     ref.segment_write(0, path, {"a": ([1, 2, 3], [1, 1, 2]), "ab": ([2], [1])})
@@ -67,7 +67,7 @@ def test_segment_without_updates_and_errors(tmp_path):
 def test_segment_reader_survives_truncated_and_corrupted_files(tmp_path):
     """the reader parses files it did not write: every truncation / byte flip must end in a TrinityError or a consistent segment,
     never in an out-of-bounds read (the process would die)"""
-    ref = load_ref()
+    ref = load_golden_ref()
     src = tmp_path / "9"
     src.mkdir()
     ref.segment_write(0, src, make_lists(3, nterms=12, ndocs=3000), ERASED, replace_below=50)

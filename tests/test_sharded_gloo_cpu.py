@@ -37,7 +37,7 @@ def _worker(rank, world, port, out):
     try:
         import torch
         import trinity_b200 as tb
-        from refharness import RefIndex, load_ref
+        from refharness import RefIndex, load_golden_ref
         from trinity_b200.sharded import concat_docs_only, gather_and_merge_topk, global_document_frequencies, shard_range
 
         lo, hi = shard_range(NDOCS, rank, world)
@@ -46,7 +46,7 @@ def _worker(rank, world, port, out):
         want_df = np.array([max(MIN_DF, NDOCS // (2 * r)) for r in range(1, NTERMS + 1)])
         assert np.array_equal(gdf, want_df), "summed shard dfs must equal the unsharded dfs"
         # the shard as an IndexSource of its own; docsCnt = GLOBAL collection size, like IndexSourcesCollectionBM25Scorer::reset
-        r = RefIndex.from_bytes(load_ref(), tb.CODEC_GOOGLE, np.asarray(s.index), None, s.names, np.asarray(s.terms), NDOCS, s.sum_hits)
+        r = RefIndex.from_bytes(load_golden_ref(), tb.CODEC_GOOGLE, np.asarray(s.index), None, s.names, np.asarray(s.terms), NDOCS, s.sum_hits)
         docs_parts, topd, tops = [], np.zeros((len(QUERIES), K), np.int32), np.full((len(QUERIES), K), -1.0, np.float32)
         for qi, q in enumerate(QUERIES):
             ids, _ = r.exec(q, False, NDOCS + 1)
